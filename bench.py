@@ -17,6 +17,9 @@ GPUs: the exact allocate loop runs as one persistent kernel per GPU whose per-st
 peer-mapped mailboxes (vc_comm_*), and the dense task x node pass (K1) is node-sharded with NCCL collectives
 (MAX all-reduce of the group statistics, all-gather + fold of the per-task best). value = placements of the one
 cluster / max-over-ranks kernel time. N scheduler replicas (one cluster per GPU) are reported as a labelled secondary number.
+
+--dump-outputs DIR writes what the last timed step returned (decisions, visits, fit errors) as DIR/<name>.npy, so that two
+builds can be compared output for output on the same seeded workload.
 """
 from __future__ import annotations
 
@@ -111,6 +114,23 @@ def run_oracle(snap, threads, want_results=False):
     return len(dec), dt
 
 
+DUMP_BYTES = 60_000_000  # keeps a dump, .npy headers included, under 64 MB
+
+
+def dump_outputs(out_dir, decisions, visits, fit_errors, job_allocated_hypernodes=None):
+    """One cycle's result as out_dir/<array>_<field>.npy in float64 (the int32 fields are exact there). Above DUMP_BYTES in
+    all, every k-th row of each array is written: the same rows for outputs of the same lengths."""
+    arrays = {f"decisions_{f}": decisions[f] for f in decisions.dtype.names}
+    arrays.update({f"visits_{f}": visits[f] for f in visits.dtype.names})
+    arrays["fit_errors"] = fit_errors
+    if job_allocated_hypernodes is not None:
+        arrays["job_allocated_hypernodes"] = job_allocated_hypernodes
+    stride = max(1, -(-8 * sum(a.size for a in arrays.values()) // DUMP_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a[::stride], np.float64))
+
+
 KERNEL_NAMES = {0: "k_commit (general)", 1: "k_commit_fast (incremental)"}
 # session shapes other than the headline one, same size (10k nodes x 100k tasks): GPU cycle vs the CPU port in the same mode
 MODE_WORKLOADS = [("Releasing resources (terminating pods: FutureIdle gradient, pipelining)", "cfg2_fut"),
@@ -195,9 +215,11 @@ def reference_arm(args, rank, world):
         run_oracle(snap, threads)
     placed, times = 0, []
     for _ in range(args.steps):
-        n, dt = run_oracle(snap, threads)
+        n, dt, out = run_oracle(snap, threads, want_results=True)
         placed += n
         times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *out)
     total = sum(times)
     val = placed / total
     line = {
@@ -251,6 +273,7 @@ def multi_gpu_arm(args, rank, world, local):
         dist.all_reduce(cnt, op=dist.ReduceOp.MAX)  # rank 0 holds the decisions of the one cluster
         placed += int(cnt[0].item())
         n_steps += int(cnt[1].item())
+    timed = res
     t_dev = sum(dev_ms) / 1e3
     # ---- e2e: host buffers -> upload on every rank -> one session -> decisions on rank 0's host ----
     torch.cuda.synchronize(); dist.barrier()
@@ -349,6 +372,8 @@ def multi_gpu_arm(args, rank, world, local):
                                           "(CUDA IPC), polled locally; no host or NCCL call inside the cycle"},
             "replicas_secondary": replicas,
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, timed.decisions, timed.visits, timed.fit_errors, timed.job_allocated_hypernodes)
         print(json.dumps(line), flush=True)
     dist.barrier()
     dist.destroy_process_group()
@@ -362,7 +387,10 @@ def main():
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--workload", default=WORKLOAD)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's result as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -413,6 +441,7 @@ def main():
         dev_ms.append(res.stats["commit_ms"])  # CUDA events on the launching stream around k_commit
         placed += len(res.decisions)
         n_steps += res.stats["n_steps"]
+    timed = res
     barrier()
     t_dev = sum(dev_ms) / 1e3
     # ---- e2e: host buffers -> upload -> allocate -> decisions on the host ------------------------
@@ -559,6 +588,8 @@ def main():
                               "us_per_placement_attempt": 1e6 * t_dev / max(1, n_steps),
                               "hbm_traffic": "inputs once (17 MB); node state is shared-memory resident"},
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, timed.decisions, timed.visits, timed.fit_errors, timed.job_allocated_hypernodes)
         print(json.dumps(line), flush=True)
         if parity is not None and not parity["placements_identical"]:
             eng.close()

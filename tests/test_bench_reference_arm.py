@@ -27,6 +27,27 @@ def test_reference_arm_line():
     assert line["e2e"] == {"value": line["value"], "unit": "pods/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+def test_reference_arm_dump_outputs(tmp_path):
+    """--dump-outputs writes the last timed step's result, one float64 .npy per field: the same arrays a direct call of the
+    oracle returns on the same seeded workload."""
+    import numpy as np
+    from oracle.pyoracle import OracleSession
+    from volcano_b200.synth import make_snapshot
+    r = _run(None, "--steps", "2", "--warmup", "0", "--dump-outputs", str(tmp_path))
+    assert r.returncode == 0, r.stderr[-2000:]
+    o = OracleSession(make_snapshot("tiny"))
+    dec, vis, fe = o.allocate()
+    o.close()
+    want = {f"decisions_{f}": dec[f] for f in dec.dtype.names}
+    want.update({f"visits_{f}": vis[f] for f in vis.dtype.names})
+    want["fit_errors"] = fe
+    assert sorted(os.listdir(tmp_path)) == sorted(f"{k}.npy" for k in want)
+    for k, a in want.items():
+        got = np.load(tmp_path / f"{k}.npy")
+        assert got.dtype == np.float64 and np.array_equal(got, a), k
+    assert len(dec) > 0
+
+
 def test_reference_arm_other_ranks_do_nothing():
     r = _run({"RANK": "1", "LOCAL_RANK": "1", "WORLD_SIZE": "2"}, "--gpus", "2", "--steps", "1", "--warmup", "0")
     assert r.returncode == 0 and not [ln for ln in r.stdout.splitlines() if ln.startswith("{")]

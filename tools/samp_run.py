@@ -1,5 +1,5 @@
 import sys, os
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from volcano_b200 import engine
 from volcano_b200.synth import make_snapshot
 snap = make_snapshot("cfg2")
