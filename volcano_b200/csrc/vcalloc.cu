@@ -60,7 +60,19 @@ constexpr size_t kMboxBytes = sizeof(uint4) * MBOX_STRIDE * 2 * 2048 * 2;
 bool g_inited = false;
 int g_device = -1;
 int g_sm_count = 0;
+int g_smem_optin = 0;  // cudaDevAttrMaxSharedMemoryPerBlockOptin of the bound device
 int g_launches = 0;
+
+// A forced or unusual launch geometry can ask for more shared memory per CTA than the device has: refuse it here, by
+// name, instead of letting cudaFuncSetAttribute fail with a bare CUDA error.
+int check_smem(const void *kfn, size_t smem, const char *what) {
+  cudaFuncAttributes a;
+  CUDA_TRY(cudaFuncGetAttributes(&a, kfn));
+  if (smem + a.sharedSizeBytes > (size_t)g_smem_optin)
+    return fail(VC_EUNSUPPORTED, "%s: %zu B of shared memory per CTA (+ %zu B static), the device allows %d B", what, smem,
+                a.sharedSizeBytes, g_smem_optin);
+  return VC_OK;
+}
 
 // Diagnostic switches: read from the environment ONCE, in vc_init (never on the per-cycle entry points), and
 // overridable at run time through vc_debug_option (tests and tools/). None of them changes a result.
@@ -446,6 +458,7 @@ int vc_init(int device) {
   CUDA_TRY(cudaGetDeviceProperties(&prop, device));
   if (!prop.cooperativeLaunch) return fail(VC_ENODEV, "device lacks cooperative launch");
   g_sm_count = prop.multiProcessorCount;
+  g_smem_optin = (int)prop.sharedMemPerBlockOptin;
   g_device = device;
   if (!g_inited) read_tunables();
   g_inited = true;
@@ -1525,6 +1538,7 @@ int vc_allocate_run(vc_snapshot *s, vc_result **out) {
                   : s->dc.to_find > 0 ? (s->topo_any ? (const void *)k_commit<true, true, true, true> : (const void *)k_commit<true, true, false, true>)
                   : s->topo_any ? (const void *)k_commit<true, true, true> : s->dc.has_future ? (s->dc.soft_active ? (const void *)k_commit<true, true> : (const void *)k_commit<true, false>)
                                      : (s->dc.soft_active ? (const void *)k_commit<false, true> : (const void *)k_commit<false, false>);
+  if (int rc = check_smem(kfn, s->smem_bytes, "commit kernel")) return rc;
   CUDA_TRY(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->smem_bytes));
   int max_blocks = 0;
   CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&max_blocks, kfn, s->block, s->smem_bytes));
@@ -2296,6 +2310,7 @@ int vc_backfill_run(vc_snapshot *s, vc_result **out) {
                     : s->dc.soft_active ? (const void *)k_backfill<true> : (const void *)k_backfill<false>;
     const size_t smem = ((sizeof(BfCtl) + 15) & ~(size_t)15) + (3 * R + 2 * K + 2) * (size_t)s->npc * 8 +
                         (size_t)s->npc * (4 + 4) + 8 + (size_t)s->npc * (8 + 4 + 1 + 1) + 8 + (size_t)G * (8 + 4 + 4) + 64;
+    if (int rc = check_smem(kfn, smem, "backfill kernel")) { delete r; return rc; }
     if ((e = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return bail(e, "backfill smem");
     int max_blocks = 0;
     if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&max_blocks, kfn, s->block, smem)) != cudaSuccess) return bail(e, "occupancy");

@@ -602,7 +602,7 @@ def encode_cluster(nodes: Sequence[Node], pods: Sequence[Pod], podgroups: Sequen
     dim_names = ["cpu", "memory"] + sorted(scalars)
     R = len(dim_names)
     if R > abi.VC_MAX_DIMS:
-        raise ValueError("too many resource dimensions")
+        raise ValueError(f"{R} resource dimensions ({', '.join(dim_names)}): the engine holds at most {abi.VC_MAX_DIMS}")
     pods_dim = dim_names.index("pods")
 
     # ---- jobs (JobID = ns/podgroup, api/job_info.go:156-164) -------------------------------
